@@ -225,6 +225,28 @@ def parity_sample(eng, params, L_row, Y_row, Z_row, P_row):
     return out
 
 
+DUMP_LIMIT = 64_000_000        # bytes --dump-outputs may write in all
+
+
+def dump_outputs(out_dir, Y, P, Z):
+    """--dump-outputs: what the last timed step returned, as <name>.npy -- Y (mel frames of this rank's utterances,
+    float32), P (the attention window position each frame was decoded with, int32 held exactly as float64) and Z
+    (linear magnitudes of every utterance this rank receives, float32).  Z exceeds DUMP_LIMIT at the default batch,
+    so it keeps a fixed, seeded sample of whole utterances, listed in Z_utterances.npy."""
+    import numpy as np
+    import torch
+    arrays = {"Y": Y.cpu().numpy(), "P": P.cpu().numpy().astype(np.float64)}
+    room = DUMP_LIMIT - sum(a.nbytes for a in arrays.values()) - 4 * 4096        # (and four .npy headers)
+    k = min(len(Z), room // (Z[0].numel() * Z.element_size() + 8))
+    if k < 1:
+        raise SystemExit("--dump-outputs: Y and P alone exceed %d bytes" % DUMP_LIMIT)
+    rows = np.sort(np.random.default_rng(0).choice(len(Z), k, replace=False))
+    arrays["Z"] = Z[torch.from_numpy(rows).to(Z.device)].cpu().numpy()
+    arrays["Z_utterances"] = rows.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_b200(args, rank, local_rank, world):
     import numpy as np
     import torch
@@ -297,6 +319,8 @@ def run_b200(args, rank, local_rank, world):
         Y, Z, P = step(marks=(evs[k][1], evs[k][2]))
         evs[k][3].record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, Y, P, Z)
     ms = sum(e[0].elapsed_time(e[3]) for e in evs)
     ms_t2m = sum(e[0].elapsed_time(e[1]) for e in evs) / args.steps
     ms_ssrn = sum(e[1].elapsed_time(e[2]) for e in evs) / args.steps
@@ -511,7 +535,15 @@ def main():
     ap.add_argument("--tensor-path", type=int, default=1, choices=[0, 1], help="1 = tcgen05 blocks (default), 0 = fp32 CUDA-core kernels only")
     ap.add_argument("--train-steps", type=int, default=5, help="timed steps of the BASELINE config 5 training step reported as train_config5 (0 = skip)")
     ap.add_argument("--train-tc", type=int, default=7, help="training GEMMs on tcgen05, bit mask (1 forward, 2 data gradient, 4 weight gradient); 0 = fp32 CUDA cores")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy "
+                    "(Y, P, a seeded utterance sample of Z; at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "b200":
+            ap.error("--dump-outputs writes the outputs of the b200 path")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE -- a minimal eager stand-in for the slice of the TensorFlow 1.x API that the
-reference's synthesis graph touches, so that the reference's OWN source files (/root/reference/modules.py,
-networks.py, train.py: Graph(mode="synthesize")) can be imported and executed in this container, where
-TensorFlow does not exist.
+reference's synthesis graph touches, so that the reference's OWN source files (modules.py, networks.py,
+train.py: Graph(mode="synthesize") of a checkout of the reference project) can be imported and executed
+without TensorFlow.  make_golden_refshim.py uses it to record the refshim_*.npz fixtures.
 
 What this pins and what it does not:
   * pinned: everything the reference's Python decides -- layer order and counts, kernel sizes, dilation
@@ -23,8 +23,6 @@ import sys
 import types
 
 import numpy as np
-
-REFERENCE = "/root/reference"
 
 
 class T(np.ndarray):
@@ -48,6 +46,7 @@ class Store:
     def __init__(self, values):
         self.values = {k: np.asarray(v) for k, v in values.items()}
         self.requested = set()
+        self.requested_shapes = {}          # name -> the shape the graph asked for (None: it named no shape)
 
     def get(self, name, shape=None):
         if name not in self.values:
@@ -56,6 +55,7 @@ class Store:
         if shape is not None and tuple(int(s) for s in shape) != v.shape:
             raise ValueError("variable %s: graph wants shape %s, store has %s" % (name, tuple(shape), v.shape))
         self.requested.add(name)
+        self.requested_shapes[name] = None if shape is None else tuple(int(s) for s in shape)
         return _t(v)
 
 
@@ -196,8 +196,9 @@ def matmul(a, b, transpose_a=False, transpose_b=False):
     return _t(a @ b)
 
 
-def install(store):
-    """Registers the stand-in modules and puts the reference on sys.path.  Returns the `tensorflow` module."""
+def install(store, reference_dir):
+    """Registers the stand-in modules and puts the reference checkout `reference_dir` on sys.path.  Returns the
+    `tensorflow` module."""
     _State.store = store
     tf = types.ModuleType("tensorflow")
     tf.float32, tf.int32, tf.int64, tf.string = np.float32, np.int32, np.int64, object
@@ -259,8 +260,8 @@ def install(store):
             m.use = lambda *a, **k: None
             sys.modules[name] = m
     sys.modules["matplotlib"].pyplot = sys.modules["matplotlib.pyplot"]
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
+    if reference_dir not in sys.path:
+        sys.path.insert(0, reference_dir)
     return tf
 
 
@@ -268,7 +269,7 @@ def run_graph(L, mels, prev_max_attentions, fetch=("Y", "max_attentions", "align
     """One `sess.run` of the reference's synthesis graph (synthesize.py:48-52): builds train.Graph with the three
     placeholders bound to these values and returns the requested attributes as plain arrays.  Unless Z is
     fetched, the SSRN call at train.py:77 is skipped (it does not feed back into Text2Mel and costs 20 GMAC)."""
-    import train as ref_train                      # /root/reference/train.py
+    import train as ref_train                      # the reference's train.py
     _State.scope = []
     _State.layer_counts = {}
     _State.feeds = [np.asarray(L, np.int32), np.asarray(mels, np.float32), np.asarray(prev_max_attentions, np.int32)]
@@ -295,7 +296,7 @@ def run_ssrn(Y):
 
 
 def synthesize(L, steps=None, with_ssrn=True):
-    """The loop of /root/reference/synthesize.py:45-57 around the reference's graph."""
+    """The loop of the reference's synthesize.py:45-57 around the reference's graph."""
     import hyperparams as ref_hp
     hp = ref_hp.Hyperparams
     L = np.asarray(L, np.int32)

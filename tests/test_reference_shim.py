@@ -1,11 +1,11 @@
-"""Parity against the REFERENCE'S OWN SOURCE.  tests/golden/refshim_*.npz were produced by importing
-/root/reference/{modules,networks,train}.py and executing Graph(mode="synthesize") under the TensorFlow API
+"""Parity against the REFERENCE'S OWN SOURCE.  tests/golden/refshim_*.npz were produced by importing the
+reference project's {modules,networks,train,data_load,utils}.py and executing them under the TensorFlow API
 stand-in tests/golden/tf_shim.py (generator: tests/golden/make_golden_refshim.py).  They pin everything the
-reference's Python decides (topology, dilations, paddings, scopes/variable names, the decoder shift, the window
-mask); the TF op semantics themselves are the shim's restatement (see its header).
+reference's Python decides (topology, dilations, paddings, scopes/variable names and shapes, the decoder shift,
+the window mask, the text adaptor, the training losses, how the vocoder composes its primitives); the TF op
+semantics themselves are the shim's restatement (see its header).
 
-  * CPU: the oracle's two restatements vs these fixtures; where /root/reference exists (this container) the
-    reference code is also executed live for a few decode steps and the variable-name schema is checked.
+  * CPU: the oracle's restatements vs these fixtures.
   * GPU: the CUDA path vs these fixtures."""
 import os
 import sys
@@ -21,7 +21,6 @@ from oracle import ref_numpy as rn
 from oracle import ref_torch as rt
 
 TOL = 1e-3            # north_star: max-abs on mel / linear magnitudes
-HAVE_REF = os.path.isfile("/root/reference/networks.py")
 
 
 @pytest.fixture(scope="module")
@@ -70,29 +69,29 @@ def test_oracle_synthesis_loop_vs_reference_code():
     assert np.abs(g["Z_sub"] - g0["Z_sub"]).max() < 1e-4
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference is not present on this machine")
 def test_reference_code_live_few_steps(P):
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import tf_shim
-    store = tf_shim.Store(P)
-    tf_shim.install(store)
+    """Three steps of the reference's loop on a batch of two and its SSRN on the first 8 frames (refshim_few_steps.npz)
+    vs the oracle's literal schedule, and the variables the reference's graphs asked for vs the parameter schema."""
+    g = golden("refshim_few_steps.npz")
     L = synthetic_text(2, 40, seed=5)
-    r = tf_shim.synthesize(L, steps=3, with_ssrn=False)
     with torch.no_grad():
         o = rt.synthesize(P, L, steps=3, literal=True, record=True)
-    assert np.abs(r["Y"][:, :3] - o["Y"].numpy()[:, :3]).max() < 2e-5
-    assert np.array_equal(r["p_hist"], o["p_hist"].numpy()[:, :3])
-    _, z = tf_shim.run_ssrn(r["Y"][:, :8])
-    _, z2 = rt.SSRN(P, torch.from_numpy(r["Y"][:, :8].copy()))
-    assert np.abs(z - z2.numpy()).max() < 2e-5
+    assert np.abs(g["Y"][:, :3] - o["Y"].numpy()[:, :3]).max() < 2e-5
+    assert np.array_equal(g["p_hist"], o["p_hist"].numpy()[:, :3])
+    _, z2 = rt.SSRN(P, torch.from_numpy(g["Y"]))
+    assert np.abs(g["Z"] - z2.numpy()).max() < 2e-5
     # the graph asked for exactly the variables of the schema (SURVEY.md App. C), with the schema's shapes
-    assert store.requested == set(P)
-    # an unknown or mis-shaped variable is an error, not a silent default
-    bad = dict(P); bad["Text2Mel/TextEnc/C_2/conv1d/kernel"] = np.zeros((1, 128, 511), np.float32)
-    tf_shim.install(tf_shim.Store(bad))
+    requested = {str(n): tuple(int(s) for s in str(sh).split(",")) for n, sh in zip(g["names"], g["shapes"])}
+    assert requested == {n: v.shape for n, v in P.items()}
+    # an unknown or mis-shaped variable is an error of the shim that recorded them, not a silent default
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    import tf_shim
+    name = "Text2Mel/TextEnc/C_2/conv1d/kernel"
+    bad = dict(P); bad[name] = np.zeros((1, 128, 511), np.float32)
     with pytest.raises(ValueError):
-        tf_shim.run_graph(L, np.zeros((2, hp.max_T, hp.n_mels), np.float32), np.zeros(2, np.int32))
-    tf_shim.install(store)
+        tf_shim.Store(bad).get(name, requested[name])
+    with pytest.raises(KeyError):
+        tf_shim.Store(P).get(name + "_1", requested[name])
 
 
 # ------------------------------------------------------------------------------------------- GPU
@@ -127,71 +126,49 @@ def test_cuda_synthesis_vs_reference_code(engine):
 
 
 # ------------------------------------------------------------------------------------------- host-side pieces
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference is not present on this machine")
-def test_text_adaptor_vs_reference_code(monkeypatch):
-    """data_load.load_data("synthesize") of the reference itself (data_load.py:79-86) on its own harvard_sentences.txt
-    vs the mirror in dc_tts_b200/data_load.py: all 20 sentences, every id."""
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import tf_shim
-    tf_shim.install(tf_shim.Store({}))
-    import data_load as ref_dl
-    import hyperparams as ref_hp
-    monkeypatch.setattr(ref_hp.Hyperparams, "test_data", "/root/reference/harvard_sentences.txt")
-    ref = ref_dl.load_data("synthesize")
+def test_text_adaptor_vs_reference_code():
+    """data_load.load_data("synthesize") of the reference itself (data_load.py:79-86) on its own harvard_sentences.txt,
+    and its load_vocab() (refshim_host.npz), vs the mirror in dc_tts_b200/data_load.py: all 20 sentences, every id."""
+    g = golden("refshim_host.npz")
+    ref = g["harvard_L"]
     from dc_tts_b200.data_load import load_data, load_vocab
     mine = load_data("synthesize", os.path.join(ROOT, "harvard_sentences.txt"))
     assert ref.shape == (20, hp.max_N) and ref.dtype == np.int32
     assert np.array_equal(ref, mine)
-    assert ref_dl.load_vocab() == load_vocab()
+    vocab = str(g["vocab"])
+    assert load_vocab() == ({c: int(i) for c, i in zip(vocab, g["vocab_index"])}, dict(enumerate(vocab)))
     assert np.array_equal(golden("refshim_synth_harvard1.npz")["L"], ref[:1])
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference is not present on this machine")
 def test_training_constants_vs_reference_code():
-    """utils.guided_attention (utils.py:134-140) and the Noam schedule (utils.py:141-145) of the reference itself."""
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import tf_shim
-    tf_shim.install(tf_shim.Store({}))
-    import utils as ref_utils
+    """utils.guided_attention (utils.py:134-140) and the Noam schedule (utils.py:141-145) of the reference itself
+    (refshim_host.npz)."""
     from oracle import ref_train as rtr
-    np.testing.assert_allclose(ref_utils.guided_attention(), rtr.guided_attention(), rtol=0, atol=1e-7)
-    for gs in (0, 1, 3999, 4000, 123456):
-        assert float(ref_utils.learning_rate_decay(hp.lr, gs)) == pytest.approx(rtr.learning_rate(gs), rel=1e-6)
+    g = golden("refshim_host.npz")
+    np.testing.assert_allclose(g["guided_attention"], rtr.guided_attention(), rtol=0, atol=1e-7)
+    assert list(g["lr_steps"]) == [0, 1, 3999, 4000, 123456]
+    for gs, lr in zip(g["lr_steps"], g["lr"]):
+        assert float(lr) == pytest.approx(rtr.learning_rate(int(gs)), rel=1e-6)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference is not present on this machine")
 def test_vocoder_and_feature_composition_vs_reference_code(monkeypatch):
-    """utils.spectrogram2wav / get_spectrograms / load_spectrograms of the reference itself, with the absent `librosa`
-    replaced by the restated primitives (oracle/ref_vocoder.py, ref_features.py): pins how the reference COMPOSES
-    them (de-normalisation, power, Griffin-Lim loop, lfilter, trim; pre-emphasis, mel, dB, normalisation, reduction) --
-    the primitives themselves stay a restatement."""
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import types
-    import tf_shim
-    tf_shim.install(tf_shim.Store({}))
-    import utils as ref_utils
+    """utils.spectrogram2wav / get_spectrograms / load_spectrograms of the reference itself (refshim_vocoder.npz), run
+    with the absent `librosa` replaced by the restated primitives (oracle/ref_vocoder.py, ref_features.py): pins how
+    the reference COMPOSES them (de-normalisation, power, Griffin-Lim loop, lfilter, trim; pre-emphasis, mel, dB,
+    normalisation, reduction) -- the primitives themselves stay a restatement."""
     from oracle import ref_features as rf
     from oracle import ref_vocoder as rv
-    lib = types.SimpleNamespace(
-        stft=lambda y, n_fft=None, hop_length=None, win_length=None: rv.stft(np.asarray(y, np.float32), n_fft, hop_length, win_length),
-        istft=lambda S, hop_length=None, win_length=None, window="hann": rv.istft(S, hop_length, win_length),
-        effects=types.SimpleNamespace(trim=lambda y: (lambda se: (y[se[0]:se[1]], se))(rv.trim_indices(np.asarray(y)))),
-        filters=types.SimpleNamespace(mel=lambda sr, n_fft, n_mels: rf.mel_basis(sr, n_fft, n_mels)),
-        load=lambda fpath, sr=None: (WAVS[fpath], sr))
-    monkeypatch.setattr(ref_utils, "librosa", lib)
-    import hyperparams as ref_hp
-    monkeypatch.setattr(ref_hp.Hyperparams, "n_iter", 3)
+    g = golden("refshim_vocoder.npz")
     monkeypatch.setattr(hp, "n_iter", 3)
     rng = np.random.default_rng(0)
     mag = rng.uniform(0.2, 0.8, (40, 1 + hp.n_fft // 2)).astype(np.float32)
-    ref_wav = ref_utils.spectrogram2wav(mag)
+    ref_wav = g["wav"]
     mine, _, _ = rv.spectrogram2wav(mag, n_iter=3)
     assert ref_wav.shape == mine.shape and np.abs(ref_wav - mine).max() <= 1e-6 * max(1.0, np.abs(mine).max())
     t = np.arange(int(hp.sr * 0.8)) / hp.sr
     y = (0.2 * np.sin(2 * np.pi * 300 * t) + 0.02 * rng.standard_normal(t.size)).astype(np.float32)
     y[:2000] *= 1e-5
-    WAVS = {"LJ001-0001.wav": y}
-    fname, mel, mg = ref_utils.load_spectrograms("LJ001-0001.wav")
+    fname, mel, mg = str(g["fname"]), g["mel"], g["mag"]
     mel2, mg2 = rf.load_spectrograms(y)
     assert fname == "LJ001-0001.wav" and mel.shape == mel2.shape and mg.shape == mg2.shape
     assert np.abs(mel - mel2).max() < 1e-6 and np.abs(mg - mg2).max() < 1e-6

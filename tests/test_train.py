@@ -1,20 +1,15 @@
 """One Text2Mel training step (BASELINE config 5; reference train.py mode "train", num=1).
-CPU: the autograd oracle against the reference's OWN training graph executed under the TF API stand-in (losses with
-the shared deterministic dropout mask), optimiser arithmetic.  GPU: CUDA losses, every gradient, and the Adam update
-against the oracle."""
-import os
-import sys
-
+CPU: the autograd oracle against the losses of the reference's OWN training graph executed under the TF API stand-in
+with the shared deterministic dropout mask (tests/golden/refshim_train_losses.npz, written by make_golden_refshim.py),
+optimiser arithmetic.  GPU: CUDA losses, every gradient, and the Adam update against the oracle."""
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import golden
 from dc_tts_b200.hyperparams import Hyperparams as hp
 from dc_tts_b200.params import init_params, synthetic_text
 from oracle import ref_train as rtr
-
-HAVE_REF = os.path.isfile("/root/reference/train.py")
 
 
 def _batch(B, seed=3):
@@ -41,45 +36,31 @@ def test_schedule_and_guided_attention():
     assert abs(W[90, 0] - (1 - np.exp(-(0.5 ** 2) / 0.08))) < 1e-6
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference is not present on this machine")
 def test_oracle_losses_vs_reference_training_graph():
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import tf_shim
+    g = golden("refshim_train_losses.npz")
     P = init_params(0, "perturbed")
-    tf_shim.install(tf_shim.Store(P))
     L, mels = _batch(2)
-    for seed, rate in ((11, hp.dropout_rate), (0, 0.0)):
-        import hyperparams as ref_hp
-        ref_hp.Hyperparams.dropout_rate = rate
-        try:
-            hook = lambda x, r, i: x * rtr.dropout_keep(x.shape, i, seed, r)
-            ref, ncalls = tf_shim.run_train_graph(L, mels, hook)
-        finally:
-            ref_hp.Hyperparams.dropout_rate = 0.05
+    assert list(g["t2m_seeds"]) == [11, 0] and list(g["t2m_rates"]) == [hp.dropout_rate, 0.0]
+    for (seed, rate), losses, ncalls in zip(((11, hp.dropout_rate), (0, 0.0)), g["t2m_losses"], g["t2m_dropout_calls"]):
         assert ncalls == (38 if rate > 0 else 0)                                       # one dropout per block
         T = {n: torch.tensor(np.asarray(P[n], np.float32)) for n in rtr.text2mel_names()}
         with torch.no_grad():
             o = rtr.forward(T, L, mels, seed, rate)
-        for k in ("loss", "loss_mels", "loss_bd1", "loss_att"):
-            assert abs(float(o[k]) - ref[k]) < 2e-6 * max(1.0, abs(ref[k])), (k, float(o[k]), ref[k])
+        for k, ref in zip(("loss", "loss_mels", "loss_bd1", "loss_att"), losses):
+            assert abs(float(o[k]) - ref) < 2e-6 * max(1.0, abs(ref)), (k, float(o[k]), ref)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference is not present on this machine")
 def test_oracle_ssrn_losses_vs_reference_training_graph():
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import tf_shim
+    g = golden("refshim_train_losses.npz")
     P = init_params(0, "perturbed")
-    tf_shim.install(tf_shim.Store(P))
     mels = np.random.default_rng(3).uniform(0, 1, (2, 12, hp.n_mels)).astype(np.float32)
     mags = np.random.default_rng(4).uniform(0, 1, (2, 48, 1 + hp.n_fft // 2)).astype(np.float32)
-    hook = lambda x, r, i: x * rtr.dropout_keep(x.shape, i, 9, r)
-    ref, ncalls = tf_shim.run_train_graph_ssrn(mels, mags, hook)
-    assert ncalls == 16
+    assert g["ssrn_dropout_calls"] == 16
     T = {n: torch.tensor(np.asarray(P[n], np.float32)) for n in rtr.ssrn_names()}
     with torch.no_grad():
         o = rtr.forward_ssrn(T, mels, mags, 9)
-    for k in ("loss", "loss_mags", "loss_bd2"):
-        assert abs(float(o[k]) - ref[k]) < 2e-6 * max(1.0, abs(ref[k])), (k, float(o[k]), ref[k])
+    for k, ref in zip(("loss", "loss_mags", "loss_bd2"), g["ssrn_losses"]):
+        assert abs(float(o[k]) - ref) < 2e-6 * max(1.0, abs(ref)), (k, float(o[k]), ref)
 
 
 def test_oracle_step_arithmetic():
