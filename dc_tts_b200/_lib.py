@@ -50,6 +50,11 @@ SIGNATURES = {
     "dctts_train_apply": (C.c_int, [Handle, _i64, C.c_float, _p]),
     "dctts_train_init_ssrn": (C.c_int, [Handle, _i32, _i32, C.c_float]),
     "dctts_train_step_ssrn": (C.c_int, [Handle, _p, _p, _i32, _i64, C.c_uint32, C.c_float, _i32, C.POINTER(C.c_float), _p]),
+    "dctts_train_step_shaped": (C.c_int, [Handle, _p, _i32, _p, _i32, _i32, _i64, C.c_uint32, C.c_float, _i32,
+                                          C.POINTER(C.c_float), _p]),
+    "dctts_train_step_ssrn_shaped": (C.c_int, [Handle, _p, _p, _i32, _i32, _i64, C.c_uint32, C.c_float, _i32,
+                                               C.POINTER(C.c_float), _p]),
+    "dctts_train_reserve": (C.c_int, [Handle, _i32, _i32]),
     "dctts_train_grads": (C.c_int, [Handle, C.POINTER(_p), C.POINTER(_i64)]),
     "dctts_train_tensor": (C.c_int, [Handle, C.c_char_p, _i32, _p, _i64]),
     "dctts_train_set_tensor": (C.c_int, [Handle, C.c_char_p, _i32, _p, _i64]),

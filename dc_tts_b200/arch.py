@@ -12,6 +12,10 @@ from collections import namedtuple
 
 from .hyperparams import Hyperparams as hp
 
+# Most characters (attention keys) per utterance the CUDA attention kernels hold (keys padded to 3 x 64); a training batch
+# with longer text fails in the library and is skipped by the trainer loop.
+ATTENTION_KEY_CAPACITY = 192
+
 # kind: "C" | "HC" | "D";  act: None | "relu";  pad: "SAME" | "CAUSAL"
 Layer = namedtuple("Layer", "kind scope cin cout size rate pad act")
 

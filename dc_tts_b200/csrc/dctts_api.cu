@@ -137,6 +137,7 @@ struct dctts_handle_s {
     struct TrainTensor { float* p; float* g; float* m; float* v; long long n; int layout, d0, d1, d2, ld; };
     struct {
         bool ready = false; int B = 0, num = 1, T_in = 0; float rate = 0.f;
+        int cap_N = 0, cap_T = 0;                               // the activation workspace holds steps up to (cap_N keys, cap_T frames)
         std::vector<TrainLayer> layers;
         std::map<std::string, TrainTensor> tensors;            // by TF variable name
         DevBuf pre, out, emb, R, align, dS, gbuf[4], dy, wT, zeros, gts, sums, ids, grads, mom, vel, entries;
@@ -1188,9 +1189,88 @@ void ensure_scratch(H* h, size_t bytes) {
 // ---------------------------------------------------------------------------- training
 // One optimiser step of the reference's trainers (train.py mode "train"): num = 1 Text2Mel (graph :43-68, losses :83-99),
 // num = 2 SSRN on ground-truth mels (:69-72, losses :100-108); Adam + clipping :122-132 -- fixed-size batches (BASELINE
-// config 5).  Forward = the fp32 block kernels with every pre-LN tensor kept; backward = kernels_train.cu.  Gradients, Adam
+// config 5) or length buckets at their own shape (data_load.py:122-129).  Forward = the fp32 block kernels with every pre-LN tensor kept; backward = kernels_train.cu.  Gradients, Adam
 // moments and the pointers of all trained variables live in three arenas with identical offsets (the gradient arena is
 // what a data-parallel all-reduce sums).  Activation / gradient rows use a leading dimension rounded to 4 floats (F = 1025).
+// Per-step geometry: TextEnc runs over N rows, AudioEnc / AudioDec over T (Text2Mel), SSRN over T doubling at every
+// transposed-conv block.  Only the row counts change from step to step; the buffers stay at their capacity offsets.
+void train_set_geometry(H* h, int N, int T) {
+    auto& tr = h->tr;
+    const int nets = tr.num == 1 ? 3 : 1;
+    for (int net = 0; net < nets; ++net) {
+        int L = (tr.num == 1 && net == 0) ? N : T;
+        for (int i = tr.first[net]; i <= tr.last[net]; ++i) {
+            auto& t = tr.layers[i];
+            t.L_in = L;
+            if (t.l->kind == K_D) L *= 2;
+            t.L = L; t.rows = (long long)tr.B * L;
+        }
+    }
+}
+
+// Activation workspace for steps of up to N keys (Text2Mel; ignored for SSRN) and T frames: the saved pre-LN tensors and
+// block outputs, the gradient ping-pong buffers, the embedding, attention context / probabilities / score gradients and
+// the tcgen05 operand planes.  Each layer's pre / out sits at the offset of the capacity shape.  Nothing here depends on
+// the shape of the trained variables: the gradient / Adam / parameter arenas and the Adam entry table are untouched, so
+// growing the workspace keeps the optimiser state.
+void train_alloc_activations(H* h, int N, int T) {
+    auto& tr = h->tr;
+    const dctts_hparams& hp = h->hp;
+    const int B = tr.B, d = hp.d;
+    train_set_geometry(h, N, T);
+    size_t pre_f = 0, out_f = 0, g_f = 0, dy_f = 0, tca_f = 0, tcb_f = 0;
+    for (auto& t : tr.layers) {
+        const LayerDev& l = *t.l;
+        pre_f += (size_t)t.rows * l.ldw; out_f += (size_t)t.rows * t.ld_out;
+        g_f = std::max(g_f, (size_t)t.rows * std::max(t.ld_out, roundup(l.cin, 4)));
+        dy_f = std::max(dy_f, (size_t)t.rows * l.ldw);
+        {   // operand planes of the tensor-core GEMMs: activations / gradients (plain and transposed), packed weights
+            const size_t rows_in = (size_t)B * t.L_in, cmax = (size_t)roundup(std::max(l.cin, l.ldw), 8);
+            tca_f = std::max(tca_f, std::max(rows_in * cmax, (size_t)l.size * B * roundup(l.cin, 8) * roundup(t.L_in, 8)));
+            tcb_f = std::max(tcb_f, std::max((size_t)B * cmax * roundup(t.L_in, 8),
+                                             (size_t)l.size * roundup(std::max(l.cin, l.ldw) + 255, 256) * roundup(std::max(l.cin, l.ldw), 32)));
+        }
+    }
+    tr.pre.ensure(pre_f * sizeof(float)); tr.out.ensure(out_f * sizeof(float));
+    if (tr.num == 1) {
+        tr.emb.ensure((size_t)B * N * hp.e * sizeof(float)); tr.R.ensure((size_t)B * T * 2 * d * sizeof(float));
+        tr.align.ensure((size_t)B * N * T * sizeof(float)); tr.dS.ensure((size_t)B * T * N * sizeof(float));
+        g_f = std::max(g_f, (size_t)B * std::max(N, T) * (size_t)std::max(2 * d, hp.e));
+    }
+    for (auto& g : tr.gbuf) g.ensure(g_f * sizeof(float));
+    tr.dy.ensure(dy_f * sizeof(float));
+    tr.tc_a_hi.ensure(tca_f * sizeof(__half)); tr.tc_a_lo.ensure(tca_f * sizeof(__half));
+    tr.tc_b_hi.ensure(tcb_f * sizeof(__half)); tr.tc_b_lo.ensure(tcb_f * sizeof(__half));
+    tr.tc.a_hi = tr.tc_a_hi.as<__half>(); tr.tc.a_lo = tr.tc_a_lo.as<__half>(); tr.tc.a_elems = tca_f;
+    tr.tc.b_hi = tr.tc_b_hi.as<__half>(); tr.tc.b_lo = tr.tc_b_lo.as<__half>(); tr.tc.b_elems = tcb_f;
+    float* pre = tr.pre.as<float>(); float* out = tr.out.as<float>();
+    for (auto& t : tr.layers) {
+        t.pre = pre; pre += (size_t)t.rows * t.l->ldw;
+        t.out = out; out += (size_t)t.rows * t.ld_out;
+    }
+    // inputs: each block reads the previous block's output; the first block of a network reads the embedding (TextEnc), the
+    // mels shifted by one frame (AudioEnc, train.py:51; set per step), R (AudioDec) or the ground-truth mels (SSRN, per step)
+    const int nets = tr.num == 1 ? 3 : 1;
+    for (int net = 0; net < nets; ++net)
+        for (int i = tr.first[net] + 1; i <= tr.last[net]; ++i) tr.layers[i].in = tr.layers[i - 1].out;
+    if (tr.num == 1) {
+        tr.layers[tr.first[0]].in = tr.emb.as<float>();
+        tr.layers[tr.first[2]].in = tr.R.as<float>();
+    }
+    tr.cap_N = tr.num == 1 ? N : 0; tr.cap_T = T;
+}
+
+// Grows the activation workspace to hold (N, T) if it does not yet; waits for the device first (the old buffers may be
+// in use by queued work).
+void train_reserve(H* h, int N, int T) {
+    auto& tr = h->tr;
+    REQUIRE(tr.ready, "dctts_train_reserve: call dctts_train_init / dctts_train_init_ssrn first");
+    if (tr.num == 2) N = 0;
+    if (N <= tr.cap_N && T <= tr.cap_T) return;
+    CUDA_CHECK(cudaDeviceSynchronize());
+    train_alloc_activations(h, std::max(N, tr.cap_N), std::max(T, tr.cap_T));
+}
+
 void train_init(H* h, int B, float rate, int num, int T_in) {
     REQUIRE(h->committed, "dctts_train_init: parameters must be committed first");
     REQUIRE(B >= 1 && rate >= 0.f && rate < 1.f && (num == 1 || num == 2) && T_in >= 1, "dctts_train_init: bad arguments");
@@ -1206,7 +1286,7 @@ void train_init(H* h, int B, float rate, int num, int T_in) {
     tr.layers.clear(); tr.tensors.clear();
     std::vector<std::vector<LayerDev>*> nets;
     if (num == 1) nets = {&h->textenc, &h->audioenc, &h->audiodec}; else nets = {&h->ssrn};
-    size_t pre_f = 0, out_f = 0, g_f = 0, dy_f = 0, wt_f = 0, tca_f = 0, tcb_f = 0;
+    size_t wt_f = 0;
     long long n_grad = 0;
     auto reserve = [&](long long n) { long long o = n_grad; n_grad += (n + 3) / 4 * 4; return o; };
     struct Off { long long W, bias, g1, b1, g2, b2; };
@@ -1215,22 +1295,10 @@ void train_init(H* h, int B, float rate, int num, int T_in) {
     int li = 0;
     for (size_t net = 0; net < nets.size(); ++net) {
         tr.first[net] = li;
-        int L = (num == 1 && net == 0) ? N : T;
         for (auto& l : *nets[net]) {
             H::TrainLayer t;
-            t.l = &l; t.li = li++; t.L_in = L;
-            if (l.kind == K_D) L *= 2;
-            t.L = L; t.rows = (long long)B * L; t.ld_out = roundup(l.cout, 4);
-            pre_f += (size_t)t.rows * l.ldw; out_f += (size_t)t.rows * t.ld_out;
-            g_f = std::max(g_f, (size_t)t.rows * std::max(t.ld_out, roundup(l.cin, 4)));
-            dy_f = std::max(dy_f, (size_t)t.rows * l.ldw);
+            t.l = &l; t.li = li++; t.ld_out = roundup(l.cout, 4);
             wt_f = std::max(wt_f, (size_t)l.size * l.ldw * roundup(l.cin, 4));
-            {   // operand planes of the tensor-core GEMMs: activations / gradients (plain and transposed), packed weights
-                const size_t rows_in = (size_t)B * t.L_in, cmax = (size_t)roundup(std::max(l.cin, l.ldw), 8);
-                tca_f = std::max(tca_f, std::max(rows_in * cmax, (size_t)l.size * B * roundup(l.cin, 8) * roundup(t.L_in, 8)));
-                tcb_f = std::max(tcb_f, std::max((size_t)B * cmax * roundup(t.L_in, 8),
-                                                 (size_t)l.size * roundup(std::max(l.cin, l.ldw) + 255, 256) * roundup(std::max(l.cin, l.ldw), 32)));
-            }
             Off o{};
             o.W = reserve((long long)l.size * l.cin * l.ldw); o.bias = reserve(l.ldw);
             o.g1 = reserve(l.cout); o.b1 = reserve(l.cout);
@@ -1240,22 +1308,14 @@ void train_init(H* h, int B, float rate, int num, int T_in) {
         }
         tr.last[net] = li - 1;
     }
-    tr.pre.ensure(pre_f * sizeof(float)); tr.out.ensure(out_f * sizeof(float));
-    if (num == 1) {
-        tr.emb.ensure((size_t)B * N * hp.e * sizeof(float)); tr.R.ensure((size_t)B * T * 2 * d * sizeof(float));
-        tr.align.ensure((size_t)B * N * T * sizeof(float)); tr.dS.ensure((size_t)B * T * N * sizeof(float));
-        g_f = std::max(g_f, (size_t)B * std::max(N, T) * (size_t)std::max(2 * d, hp.e));
-        tr.gts.ensure((size_t)N * T * sizeof(float)); launch_guided_attention(tr.gts.as<float>(), N, T, h->stream);
-    }
-    for (auto& g : tr.gbuf) g.ensure(g_f * sizeof(float));
-    tr.dy.ensure(dy_f * sizeof(float)); tr.wT.ensure(wt_f * sizeof(float));
-    tr.zeros.ensure(4096 * sizeof(float)); CUDA_CHECK(cudaMemset(tr.zeros.p, 0, 4096 * sizeof(float)));
-    tr.tc_a_hi.ensure(tca_f * sizeof(__half)); tr.tc_a_lo.ensure(tca_f * sizeof(__half));
-    tr.tc_b_hi.ensure(tcb_f * sizeof(__half)); tr.tc_b_lo.ensure(tcb_f * sizeof(__half));
-    tr.tc_slots.ensure(2048 * sizeof(unsigned));
+    tr.B = B; tr.num = num;
     tr.tc = GemmTcWs{};
-    tr.tc.a_hi = tr.tc_a_hi.as<__half>(); tr.tc.a_lo = tr.tc_a_lo.as<__half>(); tr.tc.a_elems = tca_f;
-    tr.tc.b_hi = tr.tc_b_hi.as<__half>(); tr.tc.b_lo = tr.tc_b_lo.as<__half>(); tr.tc.b_elems = tcb_f;
+    tr.cap_N = tr.cap_T = 0;
+    train_alloc_activations(h, N, T);
+    if (num == 1) { tr.gts.ensure((size_t)N * hp.max_T * sizeof(float)); launch_guided_attention(tr.gts.as<float>(), N, hp.max_T, h->stream); }
+    tr.wT.ensure(wt_f * sizeof(float));
+    tr.zeros.ensure(4096 * sizeof(float)); CUDA_CHECK(cudaMemset(tr.zeros.p, 0, 4096 * sizeof(float)));
+    tr.tc_slots.ensure(2048 * sizeof(unsigned));
     tr.tc.slots = tr.tc_slots.as<unsigned>(); tr.tc.n_slots = 2048;
     tr.sums.ensure(4 * sizeof(double));
     tr.grads.ensure(n_grad * sizeof(float)); tr.mom.ensure(n_grad * sizeof(float)); tr.vel.ensure(n_grad * sizeof(float));
@@ -1271,11 +1331,8 @@ void train_init(H* h, int B, float rate, int num, int T_in) {
         return G + off;
     };
     if (num == 1) tr.d_table = reg("Text2Mel/TextEnc/embed_1/lookup_table", h->embed_table, table_off, (long long)hp.vocab_size * hp.e);
-    float* pre = tr.pre.as<float>(); float* out = tr.out.as<float>();
     for (size_t i = 0; i < tr.layers.size(); ++i) {
         auto& t = tr.layers[i]; LayerDev& l = *t.l; const Off& o = offs[i];
-        t.pre = pre; pre += (size_t)t.rows * l.ldw;
-        t.out = out; out += (size_t)t.rows * t.ld_out;
         const long long wn = (long long)l.size * l.cin * l.ldw;
         if (l.kind == K_D) {
             t.dW = reg(l.scope + "/conv2d_transpose/kernel", l.W, o.W, wn, 2, l.size, l.cin, l.cout, l.ldw);
@@ -1288,17 +1345,13 @@ void train_init(H* h, int B, float rate, int num, int T_in) {
         t.dg1 = reg(l.scope + n1 + "/gamma", l.g1, o.g1, l.cout); t.db1 = reg(l.scope + n1 + "/beta", l.b1, o.b1, l.cout);
         if (l.kind == K_HC) { t.dg2 = reg(l.scope + "/H2/gamma", l.g2, o.g2, l.cout); t.db2 = reg(l.scope + "/H2/beta", l.b2, o.b2, l.cout); }
     }
-    // inputs: each block reads the previous block's output; the first block of a network reads the embedding (TextEnc), the
-    // mels shifted by one frame (AudioEnc, train.py:51; set per step), R (AudioDec) or the ground-truth mels (SSRN, per step)
+    // leading dimensions of the blocks' inputs (the pointers are set by train_alloc_activations and, for the mels, per step)
     for (size_t net = 0; net < nets.size(); ++net)
-        for (int i = tr.first[net]; i <= tr.last[net]; ++i) {
-            auto& t = tr.layers[i];
-            if (i > tr.first[net]) { t.in = tr.layers[i - 1].out; t.ld_in = tr.layers[i - 1].ld_out; }
-        }
+        for (int i = tr.first[net] + 1; i <= tr.last[net]; ++i) tr.layers[i].ld_in = tr.layers[i - 1].ld_out;
     if (num == 1) {
-        tr.layers[tr.first[0]].in = tr.emb.as<float>(); tr.layers[tr.first[0]].ld_in = hp.e;
+        tr.layers[tr.first[0]].ld_in = hp.e;
         tr.layers[tr.first[1]].ld_in = hp.n_mels; tr.layers[tr.first[1]].extra_shift = -1; tr.layers[tr.first[1]].need_dgrad = false;
-        tr.layers[tr.first[2]].in = tr.R.as<float>(); tr.layers[tr.first[2]].ld_in = 2 * d;
+        tr.layers[tr.first[2]].ld_in = 2 * d;
     } else {
         tr.layers[0].ld_in = hp.n_mels; tr.layers[0].need_dgrad = false;
     }
@@ -1306,7 +1359,7 @@ void train_init(H* h, int B, float rate, int num, int T_in) {
     CUDA_CHECK(cudaMemcpy(tr.entries.p, entries.data(), entries.size() * sizeof(AdamEntry), cudaMemcpyHostToDevice));
     tr.n_entries = (int)entries.size();
     CUDA_CHECK(cudaStreamSynchronize(h->stream));
-    tr.B = B; tr.rate = rate; tr.num = num; tr.T_in = T_in; tr.ready = true;
+    tr.rate = rate; tr.T_in = T_in; tr.ready = true;
 }
 
 void layer_shifts(const LayerDev& l, int extra, int* shifts) {
@@ -1429,11 +1482,19 @@ void train_read_losses(H* h, float* losses_host, double n_el, double n_att, cuda
     losses_host[0] = losses_host[1] + losses_host[2] + losses_host[3];
 }
 
-void train_forward_backward(H* h, const int* L, const float* mels, int B, uint32_t seed, float* losses_host, cudaStream_t s) {
+// Text2Mel on L (B, N) / mels (B, T, n_mels), any N <= 192 (the attention kernels' key capacity) and T: the fixed-shape
+// entry point passes (max_N, max_T), the shaped one the bucket's own extent (data_load.py:122-129, dynamic_pad=True).
+void train_forward_backward(H* h, const int* L, const float* mels, int B, int N, int T, uint32_t seed, float* losses_host,
+                            cudaStream_t s) {
     auto& tr = h->tr;
     REQUIRE(tr.ready && tr.num == 1 && tr.B == B, "dctts_train_step: call dctts_train_init with this batch size first");
+    REQUIRE(N >= 1 && T >= 1, "dctts_train_step: bad batch shape");
+    REQUIRE(N <= attn_tc_padded_keys(), "dctts_train_step: N exceeds the attention kernels' key capacity (192)");
     const dctts_hparams& hp = h->hp;
-    const int N = hp.max_N, T = hp.max_T, d = hp.d;
+    const int d = hp.d;
+    const int N_w = std::min(N, hp.max_N), T_w = std::min(T, hp.max_T);      // guided-attention window (train.py:91-95)
+    train_reserve(h, N, T);
+    train_set_geometry(h, N, T);
     Launch lc{h, s};
     CUDA_CHECK(cudaMemsetAsync(tr.grads.p, 0, tr.n_grad * sizeof(float), s));
     CUDA_CHECK(cudaMemsetAsync(tr.sums.p, 0, 4 * sizeof(double), s));
@@ -1459,20 +1520,26 @@ void train_forward_backward(H* h, const int* L, const float* mels, int B, uint32
     AttnBwdArgs ab{};
     ab.gR = gR; ab.Q = Q; ab.ldq = d; ab.K = KV; ab.V = KV + d; ab.ldkv = 2 * d; ab.align = tr.align.as<float>();
     ab.gts = tr.gts.as<float>(); ab.dS = tr.dS.as<float>(); ab.gQ = tr.gbuf[2].as<float>(); ab.gKV = tr.gbuf[3].as<float>();
-    ab.B = B; ab.T = T; ab.N = N; ab.d = d; ab.att_scale = 1.0f / ((float)B * (float)N * (float)T);
+    ab.B = B; ab.T = T; ab.N = N; ab.d = d; ab.att_scale = 1.0f / ((float)B * (float)N_w * (float)T_w);
+    ab.ld_gts = hp.max_T; ab.N_w = N_w; ab.T_w = T_w;
     launch_attn_bwd(ab, tr.sums.as<double>(), s); lc.count(3);
     float* free_a = (gR == tr.gbuf[0].as<float>()) ? tr.gbuf[1].as<float>() : tr.gbuf[0].as<float>();
     train_bwd(h, lc, tr.first[1], tr.last[1], B, seed, tr.gbuf[2].as<float>(), free_a);
     float* gEmb = train_bwd(h, lc, tr.first[0], tr.last[0], B, seed, tr.gbuf[3].as<float>(), free_a);
     launch_embed_bwd(L, gEmb, tr.d_table, B * N, hp.e, s); lc.count();
     CUDA_CHECK(cudaGetLastError());
-    train_read_losses(h, losses_host, (double)B * T * hp.n_mels, (double)B * N * T, s);
+    train_read_losses(h, losses_host, (double)B * T * hp.n_mels, (double)B * N_w * T_w, s);
 }
 
 // SSRN (num = 2): ground-truth mels in, L1 + binary divergence against the linear magnitudes (train.py:100-108)
-void train_forward_backward_ssrn(H* h, const float* mels, const float* mags, int B, uint32_t seed, float* losses_host, cudaStream_t s) {
+// mels (B, T, n_mels) -> mags (B, 4T, F); the fixed-shape entry point passes the T of dctts_train_init_ssrn
+void train_forward_backward_ssrn(H* h, const float* mels, const float* mags, int B, int T, uint32_t seed, float* losses_host,
+                                 cudaStream_t s) {
     auto& tr = h->tr;
     REQUIRE(tr.ready && tr.num == 2 && tr.B == B, "dctts_train_step_ssrn: call dctts_train_init_ssrn with this batch size first");
+    REQUIRE(T >= 1, "dctts_train_step_ssrn: bad batch shape");
+    train_reserve(h, 0, T);
+    train_set_geometry(h, 0, T);
     Launch lc{h, s};
     CUDA_CHECK(cudaMemsetAsync(tr.grads.p, 0, tr.n_grad * sizeof(float), s));
     CUDA_CHECK(cudaMemsetAsync(tr.sums.p, 0, 4 * sizeof(double), s));
@@ -1890,8 +1957,26 @@ int dctts_train_step(dctts_handle h, const int32_t* L, const float* mels, int32_
     return guarded(h, [&] {
         REQUIRE(L && mels && B >= 1 && global_step >= 0, "dctts_train_step: bad arguments");
         cudaStream_t s = S(h, stream);
-        train_forward_backward(h, reinterpret_cast<const int*>(L), mels, B, seed, losses_host, s);
+        train_forward_backward(h, reinterpret_cast<const int*>(L), mels, B, h->hp.max_N, h->hp.max_T, seed, losses_host, s);
         if (apply) train_apply(h, global_step, lr, s);
+    });
+}
+
+int dctts_train_step_shaped(dctts_handle h, const int32_t* L, int32_t N, const float* mels, int32_t T, int32_t B, int64_t global_step,
+                            uint32_t seed, float lr, int32_t apply, float* losses_host, void* stream) {
+    return guarded(h, [&] {
+        REQUIRE(L && mels && B >= 1 && N >= 1 && T >= 1 && global_step >= 0, "dctts_train_step_shaped: bad arguments");
+        cudaStream_t s = S(h, stream);
+        train_forward_backward(h, reinterpret_cast<const int*>(L), mels, B, N, T, seed, losses_host, s);
+        if (apply) train_apply(h, global_step, lr, s);
+    });
+}
+
+int dctts_train_reserve(dctts_handle h, int32_t N, int32_t T) {
+    return guarded(h, [&] {
+        REQUIRE(N >= 0 && T >= 1, "dctts_train_reserve: bad arguments");
+        REQUIRE(!(h->tr.ready && h->tr.num == 1 && N > attn_tc_padded_keys()), "dctts_train_reserve: N exceeds the attention kernels' key capacity (192)");
+        train_reserve(h, N, T);
     });
 }
 
@@ -1915,7 +2000,17 @@ int dctts_train_step_ssrn(dctts_handle h, const float* mels, const float* mags, 
     return guarded(h, [&] {
         REQUIRE(mels && mags && B >= 1 && global_step >= 0, "dctts_train_step_ssrn: bad arguments");
         cudaStream_t s = S(h, stream);
-        train_forward_backward_ssrn(h, mels, mags, B, seed, losses_host, s);
+        train_forward_backward_ssrn(h, mels, mags, B, h->tr.T_in, seed, losses_host, s);
+        if (apply) train_apply(h, global_step, lr, s);
+    });
+}
+
+int dctts_train_step_ssrn_shaped(dctts_handle h, const float* mels, const float* mags, int32_t B, int32_t T, int64_t global_step, uint32_t seed,
+                                 float lr, int32_t apply, float* losses_host, void* stream) {
+    return guarded(h, [&] {
+        REQUIRE(mels && mags && B >= 1 && T >= 1 && global_step >= 0, "dctts_train_step_ssrn_shaped: bad arguments");
+        cudaStream_t s = S(h, stream);
+        train_forward_backward_ssrn(h, mels, mags, B, T, seed, losses_host, s);
         if (apply) train_apply(h, global_step, lr, s);
     });
 }

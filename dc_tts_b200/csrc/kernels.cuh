@@ -159,11 +159,12 @@ struct AttnBwdArgs {
     const float* gR;                   // (B,T,2d) gradient of [ctx ; Q]
     const float* Q; int ldq; const float* K; const float* V; int ldkv;
     const float* align;                // (B,N,T) probabilities of the forward pass
-    const float* gts;                  // (N,T) guided-attention weights
+    const float* gts;                  // (max_N, max_T) guided-attention weights, leading dimension ld_gts
     float* dS;                         // (B,T,N) scratch
     float* gQ;                         // (B,T,d)
     float* gKV;                        // (B,N,2d)
-    int B, T, N, d; float att_scale;   // att_scale = 1 / (B N T)
+    int B, T, N, d; float att_scale;   // att_scale = 1 / (B N_w T_w)
+    int ld_gts, N_w, T_w;              // guided-attention window: keys n < N_w, frames t < T_w (train.py:91-95)
 };
 struct AdamEntry { float* p; float* g; float* m; float* v; long long n; };
 void launch_train_dropout(float* x, long long rows, int C, int ld, const DropArgs& d, cudaStream_t s);

@@ -288,8 +288,10 @@ void launch_transpose_w(const float* W, float* WT, int ntaps, int K, int N, int 
 
 // ------------------------------------------------------------------------------------ attention backward
 // Forward (networks.py:140-153, training: no window): S = Q K^T / sqrt(d), A = softmax_n(S), ctx = A V, R = [ctx ; Q];
-// loss_att = sum |A gts| / (B N T) (train.py:91-95, fixed-size batches).  One warp per query row (b, t):
-//   dA[n] = dctx . V[n] + sign(A gts) gts[n,t] / (B N T);  dS[n] = A[n] (dA[n] - sum_m A[m] dA[m])
+// loss_att = sum_window |A gts| / (B N_w T_w) (train.py:91-95: A is padded with -1 and cut to (max_N, max_T), so only
+// n < N_w = min(N, max_N), t < T_w = min(T, max_T) count; gts is the (max_N, max_T) table, leading dimension ld_gts).
+// One warp per query row (b, t):
+//   dA[n] = dctx . V[n] + [n < N_w, t < T_w] sign(A gts) gts[n,t] / (B N_w T_w);  dS[n] = A[n] (dA[n] - sum_m A[m] dA[m])
 //   dQ = dR[d:2d] + sum_n dS[n] K[n] / sqrt(d);  dS is kept (B,T,N) for the key-side kernel.
 // d = 256 = 32 lanes x 8.
 __global__ void __launch_bounds__(128) attn_bwd_q_kernel(const AttnBwdArgs a) {
@@ -311,9 +313,11 @@ __global__ void __launch_bounds__(128) attn_bwd_q_kernel(const AttnBwdArgs a) {
         for (int i = 0; i < 8; ++i) s = fmaf(dctx[i], __ldg(v + lane * 8 + i), s);
         s = wsum(s);
         const float p = a.align[((size_t)b * a.N + n) * a.T + t];
-        const float g = a.gts[(size_t)n * a.T + t];
-        const float pg = p * g;
-        s += (pg > 0.f ? g : (pg < 0.f ? -g : 0.f)) * a.att_scale;
+        if (n < a.N_w && t < a.T_w) {
+            const float g = a.gts[(size_t)n * a.ld_gts + t];
+            const float pg = p * g;
+            s += (pg > 0.f ? g : (pg < 0.f ? -g : 0.f)) * a.att_scale;
+        }
         if (lane == 0) da[n] = s;
         dot = fmaf(p, s, dot);
     }
@@ -357,12 +361,16 @@ __global__ void __launch_bounds__(128) attn_bwd_kv_kernel(const AttnBwdArgs a) {
     for (int i = 0; i < 8; ++i) { o[lane * 8 + i] = dk[i]; o[a.d + lane * 8 + i] = dv[i]; }
 }
 
-// sums[2] += sum |A gts|
-__global__ void attn_loss_kernel(const float* __restrict__ align, const float* __restrict__ gts, double* __restrict__ sums, int B, int NT) {
+// sums[2] += sum over the window n < N_w, t < T_w of |A gts|; align (B, N, T), gts leading dimension ld_gts
+__global__ void attn_loss_kernel(const float* __restrict__ align, const float* __restrict__ gts, double* __restrict__ sums, int B, int N,
+                                 int T, int ld_gts, int N_w, int T_w) {
     __shared__ double red[8];
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     double v = 0.0;
-    if (i < (long long)B * NT) v = fabsf(align[i] * gts[i % NT]);
+    if (i < (long long)B * N * T) {
+        const int r = (int)(i % ((long long)N * T)), n = r / T, t = r - n * T;
+        if (n < N_w && t < T_w) v = fabsf(align[i] * gts[(size_t)n * ld_gts + t]);
+    }
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
     __syncthreads();
@@ -371,8 +379,9 @@ __global__ void attn_loss_kernel(const float* __restrict__ align, const float* _
 
 void launch_attn_bwd(const AttnBwdArgs& a, double* sums, cudaStream_t s) {
     if (a.d != 256 || a.N > 192) throw std::runtime_error("attention backward is built for d = 256, N <= 192");
+    if (a.N_w > a.N || a.T_w > a.T || a.T_w > a.ld_gts) throw std::runtime_error("attention backward: guided-attention window exceeds the batch");
     const long long n = (long long)a.B * a.N * a.T;
-    attn_loss_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(a.align, a.gts, sums, a.B, a.N * a.T);
+    attn_loss_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(a.align, a.gts, sums, a.B, a.N, a.T, a.ld_gts, a.N_w, a.T_w);
     attn_bwd_q_kernel<<<(a.B * a.T + 3) / 4, 128, 0, s>>>(a);
     attn_bwd_kv_kernel<<<(a.B * a.N + 3) / 4, 128, 0, s>>>(a);
 }

@@ -10,6 +10,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .arch import ATTENTION_KEY_CAPACITY
 from .hyperparams import Hyperparams as hp
 from .params import check_params
 
@@ -297,14 +298,26 @@ class Engine:
         rate = self.hp.dropout_rate if dropout_rate is None else dropout_rate
         self._check(self._lib.dctts_train_init(self._h, int(B), float(rate)), "dctts_train_init")
 
+    KEY_CAPACITY = ATTENTION_KEY_CAPACITY          # characters per utterance a training step takes (include/dctts.h)
+
     def train_step(self, L, mels, global_step=0, seed=0, lr=None, apply=True):
-        """One Text2Mel optimiser step on L (B, max_N) int32 / mels (B, max_T, n_mels): forward with dropout, losses
-        (train.py:83-99), backward, clip, Adam (train.py:122-132).  Returns {loss, loss_mels, loss_bd1, loss_att}."""
+        """One Text2Mel optimiser step on L (B, N) int32 / mels (B, T, n_mels): forward with dropout, losses
+        (train.py:83-99), backward, clip, Adam (train.py:122-132).  Returns {loss, loss_mels, loss_bd1, loss_att}.
+        (max_N, max_T) batches run the fixed-shape step; any other shape -- a length bucket of `bucketed_batches`, as the
+        reference trains on them -- runs at its own extent (N <= KEY_CAPACITY; the workspace grows as needed)."""
         L = self._i32(L); mels = self._f32(mels)
+        if L.dim() != 2 or mels.dim() != 3 or mels.shape[0] != L.shape[0] or mels.shape[2] != self.hp.n_mels:
+            raise DcttsError("train_step: L must be (B, N) and mels (B, T, n_mels); got %s, %s" % (tuple(L.shape), tuple(mels.shape)))
+        B, N = L.shape
+        T = mels.shape[1]
+        if N > self.KEY_CAPACITY:
+            raise DcttsError("train_step: N = %d characters exceeds the attention kernels' key capacity (%d)" % (N, self.KEY_CAPACITY))
         out = (C.c_float * 4)()
-        self._check(self._lib.dctts_train_step(self._h, _ptr(L), _ptr(mels), L.shape[0], int(global_step), int(seed) & 0xffffffff,
-                                               float(self.hp.lr if lr is None else lr), 1 if apply else 0, out, self._stream()),
-                    "dctts_train_step")
+        args = (int(global_step), int(seed) & 0xffffffff, float(self.hp.lr if lr is None else lr), 1 if apply else 0, out, self._stream())
+        if (N, T) == (self.hp.max_N, self.hp.max_T):
+            self._check(self._lib.dctts_train_step(self._h, _ptr(L), _ptr(mels), B, *args), "dctts_train_step")
+        else:
+            self._check(self._lib.dctts_train_step_shaped(self._h, _ptr(L), N, _ptr(mels), T, B, *args), "dctts_train_step_shaped")
         return {"loss": out[0], "loss_mels": out[1], "loss_bd1": out[2], "loss_att": out[3]}
 
     def train_init_ssrn(self, B, T=None, dropout_rate=None):
@@ -313,15 +326,30 @@ class Engine:
         rate = self.hp.dropout_rate if dropout_rate is None else dropout_rate
         self._check(self._lib.dctts_train_init_ssrn(self._h, int(B), int(self.hp.max_T if T is None else T), float(rate)),
                     "dctts_train_init_ssrn")
+        self._ssrn_T = int(self.hp.max_T if T is None else T)
 
     def train_step_ssrn(self, mels, mags, global_step=0, seed=0, lr=None, apply=True):
-        """One SSRN optimiser step on ground-truth mels / mags (train.py:69-72,100-108,122-132)."""
+        """One SSRN optimiser step on ground-truth mels (B, T, n_mels) / mags (B, 4T, F) (train.py:69-72,100-108,122-132).
+        The T given to train_init_ssrn runs the fixed-shape step; any other T runs at its own extent."""
         mels = self._f32(mels); mags = self._f32(mags)
+        if mels.dim() != 3 or mags.dim() != 3 or mags.shape[0] != mels.shape[0] or mels.shape[2] != self.hp.n_mels \
+                or mags.shape[2] != self.F or mags.shape[1] != self.hp.r * mels.shape[1]:
+            raise DcttsError("train_step_ssrn: mels must be (B, T, n_mels) and mags (B, %d T, %d); got %s, %s"
+                             % (self.hp.r, self.F, tuple(mels.shape), tuple(mags.shape)))
+        B, T = mels.shape[0], mels.shape[1]
         out = (C.c_float * 4)()
-        self._check(self._lib.dctts_train_step_ssrn(self._h, _ptr(mels), _ptr(mags), mels.shape[0], int(global_step), int(seed) & 0xffffffff,
-                                                    float(self.hp.lr if lr is None else lr), 1 if apply else 0, out, self._stream()),
-                    "dctts_train_step_ssrn")
+        args = (int(global_step), int(seed) & 0xffffffff, float(self.hp.lr if lr is None else lr), 1 if apply else 0, out, self._stream())
+        if T == getattr(self, "_ssrn_T", None):
+            self._check(self._lib.dctts_train_step_ssrn(self._h, _ptr(mels), _ptr(mags), B, *args), "dctts_train_step_ssrn")
+        else:
+            self._check(self._lib.dctts_train_step_ssrn_shaped(self._h, _ptr(mels), _ptr(mags), B, T, *args), "dctts_train_step_ssrn_shaped")
         return {"loss": out[0], "loss_mags": out[1], "loss_bd2": out[2]}
+
+    def train_reserve(self, N, T):
+        """Pre-size the training workspace for steps up to N characters and T mel frames (SSRN: N is ignored), so that
+        no later bucket has to grow it.  Growing never loses the variables, gradients or Adam moments.  On a Text2Mel
+        handle an N above KEY_CAPACITY raises DcttsError (library check)."""
+        self._check(self._lib.dctts_train_reserve(self._h, int(N), int(T)), "dctts_train_reserve")
 
     def train_apply(self, global_step, lr=None):
         self._check(self._lib.dctts_train_apply(self._h, int(global_step), float(self.hp.lr if lr is None else lr), self._stream()),

@@ -11,9 +11,11 @@ path: the whole loop on the device, replayed from a CUDA graph.
 `Graph(num, mode="train")` is the reference's training object (train.py:22-135): `num_batch`, `global_step`, `lr`, the
 losses and `train_op` are fetchable with `Session.run` exactly as train.py:148 does (`sess.run([g.global_step,
 g.train_op])`): fetching `train_op` takes the next batch of the input pipeline (data_load.get_batch -> here an iterator of
-(L, mels, mags, ...) batches, dc_tts_b200/trainer.py) and runs ONE optimiser step -- forward with dropout, the losses of
-train.py:83-113, backward, clipping, Adam with the Noam rate (train.py:120-131) -- through `Engine.train_step` /
-`train_step_ssrn`.  Plots and summaries (train.py:100-104,116-119,154-157) are out of scope.
+(L, mels, mags, ...) batches, dc_tts_b200/trainer.py: `bucketed_batches` as they come, or fixed-size batches) and runs ONE
+optimiser step at that batch's own shape -- forward with dropout, the losses of train.py:83-113, backward, clipping, Adam
+with the Noam rate (train.py:120-131) -- through `Engine.train_step` / `train_step_ssrn`.  A batch with more characters
+than the attention kernels hold (192) is skipped and counted in `skipped_batches`.  Plots and summaries
+(train.py:100-104,116-119,154-157) are out of scope.
 """
 import numpy as np
 import torch
@@ -45,7 +47,7 @@ _TRAIN = {1: ("loss", "loss_mels", "loss_bd1", "loss_att"), 2: ("loss", "loss_ma
 class Graph:
     def __init__(self, num=1, mode="train", engine=None, fused=True, batches=None, num_batch=None, global_step=0):
         """mode "synthesize": the inference graph.  mode "train" (the reference default): `num` = 1 trains Text2Mel, 2 SSRN;
-        `batches` is the input pipeline, an iterator of (L, mels, mags, ...) tuples with fixed shapes (trainer.py)."""
+        `batches` is the input pipeline, an iterator of (L, mels, mags, ...) tuples, e.g. trainer.bucketed_batches(...)."""
         if mode not in ("train", "synthesize"):
             raise ValueError("mode: 'train' or 'synthesize' (train.py:22)")
         self.char2idx, self.idx2char = load_vocab()
@@ -57,11 +59,12 @@ class Graph:
                 raise ValueError("num: 1 for Text2Mel, 2 for SSRN (train.py:24)")
             if batches is None:
                 raise ValueError("Graph(mode='train') needs `batches`: the reference reads them from data_load.get_batch(); "
-                                 "here pass trainer.fixed_size_batches(...) or bucketed batches through pad_to_fixed")
+                                 "here pass trainer.bucketed_batches(...) or trainer.fixed_size_batches(...)")
             self.batches = iter(batches)
             self.num_batch = num_batch                       # train.py:33; only used for the progress bar
             self.global_step_value = int(global_step)
             self.last = {}
+            self.skipped_batches = 0
             self._initialised = False
             for name in ("global_step", "train_op", "lr") + _TRAIN[num]:
                 setattr(self, name, Symbol(self, name))
@@ -93,7 +96,11 @@ class Graph:
         """One `sess.run` of the training graph: fetching train_op consumes a batch and applies one update."""
         from .utils import learning_rate_decay
         if "train_op" in names:
+            from .trainer import fits_key_capacity
             L, mels, mags = next(self.batches)[:3]
+            while not fits_key_capacity(L):
+                self.skipped_batches += 1
+                L, mels, mags = next(self.batches)[:3]
             if not self._initialised:
                 if self.num == 1:
                     self.engine.train_init(len(L))

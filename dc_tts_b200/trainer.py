@@ -5,17 +5,20 @@ pre-computed `mels/*.npy`, `mags/*.npy` of prepo.py (data_load.py:104-112).
 
 Batching: `bucketed_batches` restates the reference's length-bucketed, dynamically padded queue (data_load.py:88-131:
 shuffled stream, buckets by text length every 20 characters, a full bucket emits a batch padded to its own longest
-member).  The CUDA training step takes FIXED shapes (B, max_N) / (B, max_T, n_mels) / (B, 4 max_T, F) -- BASELINE
-config 5 -- so `pad_to_fixed` extends the bucket's zero padding to hp.max_N / hp.max_T (`fixed_size_batches` is the plain
-shuffled variant without buckets).  Remaining difference, documented in DESIGN.md: the reference's losses average over
-the bucket's own padded extent (train.py:85-88 have no mask), here over the fixed extent, and the non-causal TextEnc sees
-zero-INPUT positions beyond the bucket length where TF sees the edge of the tensor.
+member).  `train` takes those batches as they are and every step runs at the bucket's own shape, as the reference does:
+TextEnc and the attention over the bucket's N_b characters, the audio networks over its T_b frames, the losses averaged
+over that extent and the guided-attention term over the window n < min(N_b, max_N), t < min(T_b, max_T) (train.py:85-95);
+the SSRN trainer follows each bucket's T_b.  A bucket whose text is longer than the attention kernels' key capacity
+(192 characters) is skipped and counted.  `fixed_size_batches` (plain shuffled batches) and `pad_to_fixed` (a bucket
+padded out to hp.max_N / hp.max_T) give the fixed shapes (B, max_N) / (B, max_T, n_mels) / (B, 4 max_T, F) of BASELINE
+config 5.
 """
 import codecs
 import os
 
 import numpy as np
 
+from .arch import ATTENTION_KEY_CAPACITY
 from .data_load import load_vocab, text_normalize
 from .hyperparams import Hyperparams as hp
 
@@ -96,8 +99,8 @@ def bucketed_batches(fpaths, text_lengths, texts, B=None, seed=0, loader=_load_s
     utterances emits them as one batch, every tensor padded with zeros to the longest member of THAT batch
     (dynamic_pad=True, :128): L (B, N_b) int32, mels (B, T_b, n_mels), mags (B, 4 T_b', F).  Buckets keep their partial
     contents across epochs like the TF queue does; nothing is dropped except what never fills a bucket.
-    Yields (L, mels, mags, names, bucket).  `pad_to_fixed` turns a batch into the fixed (max_N, max_T) shapes the CUDA
-    training step takes."""
+    Yields (L, mels, mags, names, bucket); `train` takes them at that shape.  `pad_to_fixed` turns a batch into the fixed
+    (max_N, max_T) shapes of BASELINE config 5."""
     B = B or hp.B
     bounds = bucket_boundaries(text_lengths)
     pending = [[] for _ in range(len(bounds) + 1)]
@@ -127,7 +130,7 @@ def bucketed_batches(fpaths, text_lengths, texts, B=None, seed=0, loader=_load_s
 
 
 def pad_to_fixed(L, mels, mags):
-    """A bucketed batch in the fixed shapes of the CUDA training step ((B, max_N), (B, max_T, n_mels), (B, 4 max_T, F)),
+    """A bucketed batch in the fixed shapes of BASELINE config 5 ((B, max_N), (B, max_T, n_mels), (B, 4 max_T, F)),
     or None when the bucket is longer than those (the reference has no such limit while training; BASELINE config 5 fixes
     N = 180, T = 210).  Zero padding is what dynamic_pad already appended, just further."""
     B, N_b = L.shape
@@ -145,15 +148,22 @@ def checkpoint_name(logdir, gs):
     return os.path.join(logdir, "model_gs_{}".format(str(gs // 1000).zfill(3) + "k"))
 
 
+def fits_key_capacity(L):
+    """Whether a batch's text fits the attention kernels (ATTENTION_KEY_CAPACITY characters)."""
+    return np.shape(L)[1] <= ATTENTION_KEY_CAPACITY
+
+
 def train(num, engine, batches, num_iterations=None, logdir=None, global_step=None, save_every=1000, log=print, resume=True,
           rank=0, world=1, allreduce=None):
-    """train.py:137-160 for num = 1 (Text2Mel) or 2 (SSRN).  `batches` yields (L, mels, mags, names); `engine` is an
-    `Engine` with parameters loaded.  Like tf.train.Supervisor (train.py:144), a `logdir` that already holds a checkpoint
+    """train.py:137-160 for num = 1 (Text2Mel) or 2 (SSRN).  `batches` yields (L, mels, mags, names) or the
+    (L, mels, mags, names, bucket) of `bucketed_batches`, each step at its batch's own shape; a batch with more than
+    ATTENTION_KEY_CAPACITY characters is skipped (the next batch takes its step) and the number skipped is logged.
+    `engine` is an `Engine` with parameters loaded.  Like tf.train.Supervisor (train.py:144), a `logdir` that already holds a checkpoint
     is RESUMED: variables, Adam slots and the global step come back from it (`resume=False` or an explicit `global_step`
     starts over).  Data parallel (BASELINE config 5, `world` > 1): every rank feeds its own disjoint `batches`, the step
     runs with apply=False, `allreduce` (default dc_tts_b200.parallel.allreduce_mean_) averages the flat gradient arena,
     every rank applies the identical Adam update, dropout masks differ per rank (seed = gs * world + rank) and only rank 0
-    writes checkpoints.  Returns the final global step."""
+    writes checkpoints; ranks may hold buckets of different shapes in the same step.  Returns the final global step."""
     if num not in (1, 2):
         raise ValueError("num: 1 for Text2Mel, 2 for SSRN (train.py:139)")
     num_iterations = hp.num_iterations if num_iterations is None else num_iterations
@@ -161,7 +171,12 @@ def train(num, engine, batches, num_iterations=None, logdir=None, global_step=No
     os.makedirs(logdir, exist_ok=True)
     gs = int(global_step or 0)
     initialised = False
-    for L, mels, mags, _names in batches:
+    skipped = 0
+    for batch in batches:
+        L, mels, mags = batch[:3]
+        if not fits_key_capacity(L):
+            skipped += 1
+            continue
         if not initialised:
             if num == 1:
                 engine.train_init(len(L))
@@ -193,4 +208,6 @@ def train(num, engine, batches, num_iterations=None, logdir=None, global_step=No
             log("step %d  %s" % (gs, "  ".join("%s %.4f" % kv for kv in sorted(losses.items()))))
         if gs > num_iterations:                   # train.py:160
             break
+    if skipped:
+        log("skipped %d batches with more than %d characters (attention key capacity)" % (skipped, ATTENTION_KEY_CAPACITY))
     return gs

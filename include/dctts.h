@@ -171,6 +171,21 @@ int dctts_train_apply(dctts_handle h, int64_t global_step, float lr, void* strea
 int dctts_train_init_ssrn(dctts_handle h, int32_t B, int32_t T, float dropout_rate);
 int dctts_train_step_ssrn(dctts_handle h, const float* mels, const float* mags, int32_t B, int64_t global_step, uint32_t seed, float lr,
                           int32_t apply, float* losses_host, void* stream);
+/* Length-bucketed batches at their own shape, as the reference trains on them (data_load.py:122-129, dynamic_pad=True):
+ * Text2Mel on L (B, N) int32 / mels (B, T, n_mels), SSRN on mels (B, T, n_mels) / mags (B, 4T, 1 + n_fft/2), DEVICE
+ * pointers, B as given to the init call.  TextEnc and the attention keys run over N rows, the other networks over T
+ * frames; the L1 / binary-divergence losses average over the batch's own extent.  The guided-attention term covers the
+ * window n < min(N, max_N), t < min(T, max_T) of the (max_N, max_T) weight table, divided by B min(N, max_N) min(T, max_T)
+ * (train.py:91-95 pads A with -1 and cuts it to (max_N, max_T)).  N <= 192 (the attention kernels' key capacity), T is
+ * bounded by memory only.  The activation workspace grows on demand (the device is synchronised first);
+ * dctts_train_reserve pre-sizes it for steps up to (N, T) (SSRN: N is ignored).  Growth keeps the variables, gradients,
+ * Adam moments and everything dctts_train_tensor reads.  At (max_N, max_T) (SSRN: the init T) the shaped steps compute
+ * what dctts_train_step / dctts_train_step_ssrn compute. */
+int dctts_train_step_shaped(dctts_handle h, const int32_t* L, int32_t N, const float* mels, int32_t T, int32_t B,
+                            int64_t global_step, uint32_t seed, float lr, int32_t apply, float* losses_host, void* stream);
+int dctts_train_step_ssrn_shaped(dctts_handle h, const float* mels, const float* mags, int32_t B, int32_t T,
+                                 int64_t global_step, uint32_t seed, float lr, int32_t apply, float* losses_host, void* stream);
+int dctts_train_reserve(dctts_handle h, int32_t N, int32_t T);
 int dctts_train_grads(dctts_handle h, float** grads, int64_t* count);
 int dctts_train_tensor(dctts_handle h, const char* tf_name, int32_t what, float* host_out, int64_t count);
 /* Inverse of dctts_train_tensor for what = 0 (variable), 2 (Adam m), 3 (Adam v): restores a training state (resume). */
