@@ -12,8 +12,10 @@ from collections import namedtuple
 
 from .hyperparams import Hyperparams as hp
 
-# Most characters (attention keys) per utterance the CUDA attention kernels hold (keys padded to 3 x 64); a training batch
-# with longer text fails in the library and is skipped by the trainer loop.
+# Most characters (attention keys) per utterance a handle with hp.max_N <= 192 takes, as the shipped LJ hyper-parameters
+# have.  The library fixes each handle's capacity at creation, max(192, round_up(max_N, 64)) for max_N <= 512, and
+# reports it (Engine.KEY_CAPACITY); this value is the fallback for engines that do not.  A training batch with longer
+# text fails in the library and is skipped by the trainer loop.
 ATTENTION_KEY_CAPACITY = 192
 
 # kind: "C" | "HC" | "D";  act: None | "relu";  pad: "SAME" | "CAUSAL"

@@ -160,6 +160,7 @@ struct dctts_handle_s {
     int64_t ar_nodes = 0;
 
     int tensor_path = 1;          // tcgen05 blocks wherever they apply; 0 forces the fp32 CUDA-core kernels
+    int key_cap = 192;            // longest text (keys) any entry point takes: max(192, round_up(max_N, 64)), fixed at create
     int64_t launches = 0;
 
     // kernel-variant switches (dctts_set_option); the defaults are the measured-best configuration
@@ -867,7 +868,7 @@ void run_attention(Launch& lc, const float* Q, int ldq, const float* K, int ldk,
                    RowWin win, int N, const int* pma, float* R, float* align, long long* maxatt,
                    int* p_next, int* p_hist, Planes Rpl = Planes{}) {
     H* h = lc.h;
-    REQUIRE(N <= 192, "attention: N exceeds the kernel's key capacity (192)");
+    REQUIRE(N <= h->key_cap, "attention: N = " + std::to_string(N) + " exceeds the handle's key capacity (" + std::to_string(h->key_cap) + ")");
     REQUIRE(h->hp.d <= 256, "attention: d exceeds 256");
     AttnArgs a{};
     a.Q = Q; a.ldq = ldq; a.K = K; a.ldk = ldk; a.V = V; a.ldv = ldv;
@@ -880,12 +881,12 @@ void run_attention(Launch& lc, const float* Q, int ldq, const float* K, int ldk,
 
 // Full-sequence attention on the tensor cores (kernels_attn_tc.cu): dense or with the monotonic
 // window.  Q, K, V are fp32 device tensors; their split planes are built here.
-bool attention_tc_ok(H* h, int N) { return h->tensor_path == 1 && h->hp.d == 256 && N <= attn_tc_padded_keys(); }
+bool attention_tc_ok(H* h, int N) { return h->tensor_path == 1 && h->hp.d == 256 && N <= h->key_cap; }
 
 void run_attention_tc(Launch& lc, const float* Q, int ldq, const float* K, int ldk, const float* V, int ldv, int B, int T,
                       int N, const int* pma, float* R, float* align, long long* maxatt, Planes Rpl) {
     H* h = lc.h;
-    const int d = h->hp.d, NP = attn_tc_padded_keys();
+    const int d = h->hp.d, NP = attn_tc_padded_keys(N);
     const size_t need[3] = {(size_t)B * T * d * sizeof(__half), (size_t)B * N * d * sizeof(__half), (size_t)B * d * NP * sizeof(__half)};
     for (int i = 0; i < 6; ++i)
         if (h->attpl[i].bytes < need[i / 2]) { CUDA_CHECK(cudaDeviceSynchronize()); h->attpl[i].ensure(need[i / 2]); }
@@ -1482,14 +1483,14 @@ void train_read_losses(H* h, float* losses_host, double n_el, double n_att, cuda
     losses_host[0] = losses_host[1] + losses_host[2] + losses_host[3];
 }
 
-// Text2Mel on L (B, N) / mels (B, T, n_mels), any N <= 192 (the attention kernels' key capacity) and T: the fixed-shape
+// Text2Mel on L (B, N) / mels (B, T, n_mels), any N <= the handle's key capacity and any T: the fixed-shape
 // entry point passes (max_N, max_T), the shaped one the bucket's own extent (data_load.py:122-129, dynamic_pad=True).
 void train_forward_backward(H* h, const int* L, const float* mels, int B, int N, int T, uint32_t seed, float* losses_host,
                             cudaStream_t s) {
     auto& tr = h->tr;
     REQUIRE(tr.ready && tr.num == 1 && tr.B == B, "dctts_train_step: call dctts_train_init with this batch size first");
     REQUIRE(N >= 1 && T >= 1, "dctts_train_step: bad batch shape");
-    REQUIRE(N <= attn_tc_padded_keys(), "dctts_train_step: N exceeds the attention kernels' key capacity (192)");
+    REQUIRE(N <= h->key_cap, "dctts_train_step: N = " + std::to_string(N) + " exceeds the handle's key capacity (" + std::to_string(h->key_cap) + ")");
     const dctts_hparams& hp = h->hp;
     const int d = hp.d;
     const int N_w = std::min(N, hp.max_N), T_w = std::min(T, hp.max_T);      // guided-attention window (train.py:91-95)
@@ -1507,7 +1508,7 @@ void train_forward_backward(H* h, const int* L, const float* mels, int B, int N,
     const float* Q = tr.layers[tr.last[1]].out;                // (B, T, d)
     // dense softmax attention (training: no window, networks.py:140-153): the tcgen05 kernel of the synthesis path when the
     // forward GEMMs are on the tensor cores (it does not touch the weights), else one warp per query row on CUDA cores
-    if ((h->opt.train_tc & 1) && d == 256 && N <= attn_tc_padded_keys())
+    if ((h->opt.train_tc & 1) && d == 256)
         run_attention_tc(lc, Q, d, KV, 2 * d, KV + d, 2 * d, B, T, N, nullptr, tr.R.as<float>(), tr.align.as<float>(), nullptr, Planes{});
     else
         run_attention(lc, Q, d, KV, 2 * d, KV + d, 2 * d, RowWin{B, T, T, nullptr}, N, nullptr, tr.R.as<float>(), tr.align.as<float>(),
@@ -1598,10 +1599,14 @@ int dctts_create(const dctts_hparams* hp, int device, dctts_handle* out) {
         cudaDeviceProp prop;
         CUDA_CHECK(cudaGetDeviceProperties(&prop, device));
         if (prop.major != 10) throw std::runtime_error("dctts_create: this library is built for sm_100a (B200) only");
-        if (hp->d > 256 || hp->d % 8 || hp->e % 4 || hp->max_N > 192 || hp->r != 4)
+        if (hp->d > 256 || hp->d % 8 || hp->e % 4 || hp->max_N < 1 || hp->max_T < 1 || hp->r != 4)
             throw std::runtime_error("dctts_create: unsupported hyper-parameters");
+        if (hp->max_N > attn_tc_max_keys())
+            throw std::runtime_error("dctts_create: max_N = " + std::to_string(hp->max_N) + " exceeds the attention kernels' limit of " +
+                                     std::to_string(attn_tc_max_keys()) + " characters");
         std::unique_ptr<dctts_handle_s> h(new dctts_handle_s());
         h->hp = *hp; h->device = device; h->F = 1 + hp->n_fft / 2;
+        h->key_cap = attn_tc_padded_keys(hp->max_N);
         CUDA_CHECK(cudaSetDevice(device));
         CUDA_CHECK(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
         build_tables(h.get());
@@ -1975,7 +1980,8 @@ int dctts_train_step_shaped(dctts_handle h, const int32_t* L, int32_t N, const f
 int dctts_train_reserve(dctts_handle h, int32_t N, int32_t T) {
     return guarded(h, [&] {
         REQUIRE(N >= 0 && T >= 1, "dctts_train_reserve: bad arguments");
-        REQUIRE(!(h->tr.ready && h->tr.num == 1 && N > attn_tc_padded_keys()), "dctts_train_reserve: N exceeds the attention kernels' key capacity (192)");
+        REQUIRE(!(h->tr.ready && h->tr.num == 1 && N > h->key_cap),
+                "dctts_train_reserve: N = " + std::to_string(N) + " exceeds the handle's key capacity (" + std::to_string(h->key_cap) + ")");
         train_reserve(h, N, T);
     });
 }
@@ -2163,6 +2169,7 @@ int dctts_get_option(dctts_handle h, const char* name, int32_t* value) {
         REQUIRE(value, "dctts_get_option: null output");
         if (name && std::string(name) == "pdl") { *value = pdl_enabled() ? 1 : 0; return; }
         if (name && std::string(name) == "decode_available") { *value = h->dec.ok ? 1 : 0; return; }
+        if (name && std::string(name) == "key_capacity") { *value = h->key_cap; return; }
         if (name && std::string(name) == "decode_max_clusters") { *value = h->dec.max_clusters; return; }   // co-resident 16-CTA clusters
         int* slot = option_slot(h, name);
         REQUIRE(slot, "dctts_get_option: unknown option");

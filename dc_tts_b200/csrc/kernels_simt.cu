@@ -610,14 +610,15 @@ void launch_ln_rows(const LnArgs& a, cudaStream_t s) {
 // Attention (networks.py:140-153): one warp per query row.  With the monotonic window only
 // keys p <= n < p+win are live -- every other softmax term is exactly 0 in the reference
 // (mask value -2^32+1 underflows, SURVEY.md App. B) -- so only those are evaluated.
+// Each warp keeps its row's scores in N floats of dynamic shared memory.
 // ------------------------------------------------------------------------------------
-constexpr int ATT_MAXN = 192;
+constexpr int ATT_MAXN = 512;
 constexpr int ATT_WARPS = 4;
 
 __global__ void __launch_bounds__(ATT_WARPS * 32) attention_kernel(const AttnArgs a) {
     pdl_launch_dependents();
     pdl_wait();
-    __shared__ float probs[ATT_WARPS][ATT_MAXN];
+    extern __shared__ float probs[];           // [ATT_WARPS][N]
     const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int warp = blockIdx.x * ATT_WARPS + wib;
     const int R = a.win.R, T = a.win.L;
@@ -640,7 +641,7 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) attention_kernel(const AttnArg
 #pragma unroll
     for (int i = 0; i < 8; ++i) qv[i] = (lane * 8 + i < d) ? q[lane * 8 + i] : 0.f;
     const float scale = rsqrtf((float)d);    // exact for d = 256
-    float* pr = probs[wib];
+    float* pr = probs + (size_t)wib * a.N;
 
     // scores
     for (int n = n_lo; n < n_hi; ++n) {
@@ -716,7 +717,9 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) attention_kernel(const AttnArg
 void launch_attention(const AttnArgs& a, cudaStream_t s) {
     const int rows = a.win.B * a.win.R;
     if (rows <= 0) return;
-    launch_kernel(attention_kernel, dim3((rows + ATT_WARPS - 1) / ATT_WARPS), dim3(ATT_WARPS * 32), 0, s, a);
+    if (a.N < 1 || a.N > ATT_MAXN) throw std::runtime_error("attention: N must be in [1, 512]");
+    launch_kernel(attention_kernel, dim3((rows + ATT_WARPS - 1) / ATT_WARPS), dim3(ATT_WARPS * 32),
+                  (size_t)ATT_WARPS * a.N * sizeof(float), s, a);
 }
 
 // ------------------------------------------------------------------------------------

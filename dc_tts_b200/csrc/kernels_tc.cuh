@@ -76,8 +76,10 @@ struct AttnTcArgs {
     int T, N, d, win_size;
     float scale;                   // 1/sqrt(d)
 };
-int attn_tc_padded_keys();
-// K, V fp32 -> K planes (B,N,d) and transposed V planes (B,d,192), keys >= N zero
+// Keys the kernel pads N to: max(192, round_up(N, 64)); N <= attn_tc_max_keys() (512)
+int attn_tc_padded_keys(int N);
+int attn_tc_max_keys();
+// K, V fp32 -> K planes (B,N,d) and transposed V planes (B,d,vtp.ld), keys in [N, attn_tc_padded_keys(N)) zero
 void launch_attn_kv_planes(const float* K, int ldk, const float* V, int ldv, Planes kp, Planes vtp, int B, int N, int d,
                            cudaStream_t s);
 void launch_attention_tc(const Planes& Q, const Planes& K, const Planes& Vt, const AttnTcArgs& a, int B, cudaStream_t s);

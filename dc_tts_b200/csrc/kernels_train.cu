@@ -293,9 +293,10 @@ void launch_transpose_w(const float* W, float* WT, int ntaps, int K, int N, int 
 // One warp per query row (b, t):
 //   dA[n] = dctx . V[n] + [n < N_w, t < T_w] sign(A gts) gts[n,t] / (B N_w T_w);  dS[n] = A[n] (dA[n] - sum_m A[m] dA[m])
 //   dQ = dR[d:2d] + sum_n dS[n] K[n] / sqrt(d);  dS is kept (B,T,N) for the key-side kernel.
-// d = 256 = 32 lanes x 8.
+// d = 256 = 32 lanes x 8; each warp keeps dA in N floats of dynamic shared memory.
+constexpr int ATT_BWD_MAXN = 512;
 __global__ void __launch_bounds__(128) attn_bwd_q_kernel(const AttnBwdArgs a) {
-    __shared__ float sdA[4][192];
+    extern __shared__ float sdA[];              // [4][N]
     const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int row = blockIdx.x * 4 + wib;
     if (row >= a.B * a.T) return;
@@ -304,7 +305,7 @@ __global__ void __launch_bounds__(128) attn_bwd_q_kernel(const AttnBwdArgs a) {
     float dctx[8], dq[8];
 #pragma unroll
     for (int i = 0; i < 8; ++i) { dctx[i] = gR[lane * 8 + i]; dq[i] = gR[a.d + lane * 8 + i]; }
-    float* da = sdA[wib];
+    float* da = sdA + (size_t)wib * a.N;
     float dot = 0.f;
     for (int n = 0; n < a.N; ++n) {
         const float* v = a.V + ((size_t)b * a.N + n) * a.ldkv;
@@ -378,11 +379,11 @@ __global__ void attn_loss_kernel(const float* __restrict__ align, const float* _
 }
 
 void launch_attn_bwd(const AttnBwdArgs& a, double* sums, cudaStream_t s) {
-    if (a.d != 256 || a.N > 192) throw std::runtime_error("attention backward is built for d = 256, N <= 192");
+    if (a.d != 256 || a.N < 1 || a.N > ATT_BWD_MAXN) throw std::runtime_error("attention backward is built for d = 256, N <= 512");
     if (a.N_w > a.N || a.T_w > a.T || a.T_w > a.ld_gts) throw std::runtime_error("attention backward: guided-attention window exceeds the batch");
     const long long n = (long long)a.B * a.N * a.T;
     attn_loss_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(a.align, a.gts, sums, a.B, a.N, a.T, a.ld_gts, a.N_w, a.T_w);
-    attn_bwd_q_kernel<<<(a.B * a.T + 3) / 4, 128, 0, s>>>(a);
+    attn_bwd_q_kernel<<<(a.B * a.T + 3) / 4, 128, (size_t)4 * a.N * sizeof(float), s>>>(a);
     attn_bwd_kv_kernel<<<(a.B * a.N + 3) / 4, 128, 0, s>>>(a);
 }
 

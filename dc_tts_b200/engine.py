@@ -10,7 +10,6 @@ import numpy as np
 import torch
 
 from . import _lib
-from .arch import ATTENTION_KEY_CAPACITY
 from .hyperparams import Hyperparams as hp
 from .params import check_params
 
@@ -42,6 +41,8 @@ class Engine:
             raise DcttsError("dctts_create: " + self._lib.dctts_last_error(None).decode())
         self._h = h
         self.params_loaded = False
+        # characters per utterance every entry point of this handle takes: max(192, round_up(max_N, 64)) (include/dctts.h)
+        self.KEY_CAPACITY = self.get_option("key_capacity")
 
     # ------------------------------------------------------------------ plumbing
     def close(self):
@@ -190,6 +191,7 @@ class Engine:
         B, N = L.shape
         if N != self.hp.max_N:
             raise DcttsError("TextEnc: text must be padded to max_N=%d (reference networks.py:145)" % self.hp.max_N)
+        self._check_keys("textenc", N)
         K, V = self._empty(B, N, self.hp.d), self._empty(B, N, self.hp.d)
         self._check(self._lib.dctts_textenc(self._h, _ptr(L), B, _ptr(K), _ptr(V), self._stream()), "dctts_textenc")
         return K, V
@@ -239,6 +241,7 @@ class Engine:
         B = L.shape[0]
         if L.shape[1] != self.hp.max_N or mels.shape[1] != self.hp.max_T:
             raise DcttsError("synthesize graph needs N == max_N and T == max_T (reference networks.py:145)")
+        self._check_keys("text2mel_forward", L.shape[1])
         Y = self._empty(B, self.hp.max_T, self.hp.n_mels)
         M = self._empty(B, self.hp.max_T, dtype=torch.int64)
         A = self._empty(B, self.hp.max_N, self.hp.max_T) if want_alignments else None
@@ -298,7 +301,9 @@ class Engine:
         rate = self.hp.dropout_rate if dropout_rate is None else dropout_rate
         self._check(self._lib.dctts_train_init(self._h, int(B), float(rate)), "dctts_train_init")
 
-    KEY_CAPACITY = ATTENTION_KEY_CAPACITY          # characters per utterance a training step takes (include/dctts.h)
+    def _check_keys(self, what, N):
+        if N > self.KEY_CAPACITY:
+            raise DcttsError("%s: N = %d characters exceeds the attention kernels' key capacity (%d)" % (what, N, self.KEY_CAPACITY))
 
     def train_step(self, L, mels, global_step=0, seed=0, lr=None, apply=True):
         """One Text2Mel optimiser step on L (B, N) int32 / mels (B, T, n_mels): forward with dropout, losses
@@ -310,8 +315,7 @@ class Engine:
             raise DcttsError("train_step: L must be (B, N) and mels (B, T, n_mels); got %s, %s" % (tuple(L.shape), tuple(mels.shape)))
         B, N = L.shape
         T = mels.shape[1]
-        if N > self.KEY_CAPACITY:
-            raise DcttsError("train_step: N = %d characters exceeds the attention kernels' key capacity (%d)" % (N, self.KEY_CAPACITY))
+        self._check_keys("train_step", N)
         out = (C.c_float * 4)()
         args = (int(global_step), int(seed) & 0xffffffff, float(self.hp.lr if lr is None else lr), 1 if apply else 0, out, self._stream())
         if (N, T) == (self.hp.max_N, self.hp.max_T):

@@ -14,7 +14,7 @@ g.train_op])`): fetching `train_op` takes the next batch of the input pipeline (
 (L, mels, mags, ...) batches, dc_tts_b200/trainer.py: `bucketed_batches` as they come, or fixed-size batches) and runs ONE
 optimiser step at that batch's own shape -- forward with dropout, the losses of train.py:83-113, backward, clipping, Adam
 with the Noam rate (train.py:120-131) -- through `Engine.train_step` / `train_step_ssrn`.  A batch with more characters
-than the attention kernels hold (192) is skipped and counted in `skipped_batches`.  Plots and summaries
+than the engine's key capacity (Engine.KEY_CAPACITY) is skipped and counted in `skipped_batches`.  Plots and summaries
 (train.py:100-104,116-119,154-157) are out of scope.
 """
 import numpy as np
@@ -96,9 +96,9 @@ class Graph:
         """One `sess.run` of the training graph: fetching train_op consumes a batch and applies one update."""
         from .utils import learning_rate_decay
         if "train_op" in names:
-            from .trainer import fits_key_capacity
+            from .trainer import fits_key_capacity, key_capacity
             L, mels, mags = next(self.batches)[:3]
-            while not fits_key_capacity(L):
+            while not fits_key_capacity(L, key_capacity(self.engine)):
                 self.skipped_batches += 1
                 L, mels, mags = next(self.batches)[:3]
             if not self._initialised:

@@ -8,10 +8,10 @@ shuffled stream, buckets by text length every 20 characters, a full bucket emits
 member).  `train` takes those batches as they are and every step runs at the bucket's own shape, as the reference does:
 TextEnc and the attention over the bucket's N_b characters, the audio networks over its T_b frames, the losses averaged
 over that extent and the guided-attention term over the window n < min(N_b, max_N), t < min(T_b, max_T) (train.py:85-95);
-the SSRN trainer follows each bucket's T_b.  A bucket whose text is longer than the attention kernels' key capacity
-(192 characters) is skipped and counted.  `fixed_size_batches` (plain shuffled batches) and `pad_to_fixed` (a bucket
-padded out to hp.max_N / hp.max_T) give the fixed shapes (B, max_N) / (B, max_T, n_mels) / (B, 4 max_T, F) of BASELINE
-config 5.
+the SSRN trainer follows each bucket's T_b.  A bucket whose text is longer than the engine's key capacity
+(`Engine.KEY_CAPACITY`: 192 characters for hp.max_N <= 192, up to 512 as hp.max_N grows) is skipped and counted.
+`fixed_size_batches` (plain shuffled batches) and `pad_to_fixed` (a bucket padded out to hp.max_N / hp.max_T) give the
+fixed shapes (B, max_N) / (B, max_T, n_mels) / (B, 4 max_T, F) of BASELINE config 5.
 """
 import codecs
 import os
@@ -148,16 +148,21 @@ def checkpoint_name(logdir, gs):
     return os.path.join(logdir, "model_gs_{}".format(str(gs // 1000).zfill(3) + "k"))
 
 
-def fits_key_capacity(L):
-    """Whether a batch's text fits the attention kernels (ATTENTION_KEY_CAPACITY characters)."""
-    return np.shape(L)[1] <= ATTENTION_KEY_CAPACITY
+def fits_key_capacity(L, capacity=ATTENTION_KEY_CAPACITY):
+    """Whether a batch's text fits `capacity` characters (an engine's KEY_CAPACITY)."""
+    return np.shape(L)[1] <= capacity
+
+
+def key_capacity(engine):
+    """The engine's key capacity; ATTENTION_KEY_CAPACITY for an engine that does not report one."""
+    return getattr(engine, "KEY_CAPACITY", ATTENTION_KEY_CAPACITY)
 
 
 def train(num, engine, batches, num_iterations=None, logdir=None, global_step=None, save_every=1000, log=print, resume=True,
           rank=0, world=1, allreduce=None):
     """train.py:137-160 for num = 1 (Text2Mel) or 2 (SSRN).  `batches` yields (L, mels, mags, names) or the
     (L, mels, mags, names, bucket) of `bucketed_batches`, each step at its batch's own shape; a batch with more than
-    ATTENTION_KEY_CAPACITY characters is skipped (the next batch takes its step) and the number skipped is logged.
+    the engine's KEY_CAPACITY characters is skipped (the next batch takes its step) and the number skipped is logged.
     `engine` is an `Engine` with parameters loaded.  Like tf.train.Supervisor (train.py:144), a `logdir` that already holds a checkpoint
     is RESUMED: variables, Adam slots and the global step come back from it (`resume=False` or an explicit `global_step`
     starts over).  Data parallel (BASELINE config 5, `world` > 1): every rank feeds its own disjoint `batches`, the step
@@ -172,9 +177,10 @@ def train(num, engine, batches, num_iterations=None, logdir=None, global_step=No
     gs = int(global_step or 0)
     initialised = False
     skipped = 0
+    capacity = key_capacity(engine)
     for batch in batches:
         L, mels, mags = batch[:3]
-        if not fits_key_capacity(L):
+        if not fits_key_capacity(L, capacity):
             skipped += 1
             continue
         if not initialised:
@@ -209,5 +215,5 @@ def train(num, engine, batches, num_iterations=None, logdir=None, global_step=No
         if gs > num_iterations:                   # train.py:160
             break
     if skipped:
-        log("skipped %d batches with more than %d characters (attention key capacity)" % (skipped, ATTENTION_KEY_CAPACITY))
+        log("skipped %d batches with more than %d characters (attention key capacity)" % (skipped, capacity))
     return gs

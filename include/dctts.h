@@ -38,14 +38,16 @@ typedef struct dctts_hparams {
     int32_t c;                   /* hp.c = 512  */
     int32_t n_mels;              /* hp.n_mels = 80 */
     int32_t n_fft;               /* hp.n_fft = 2048 -> F = 1 + n_fft/2 */
-    int32_t max_N;               /* hp.max_N = 180 */
+    int32_t max_N;               /* hp.max_N = 180; at most 512 (see "key_capacity" below) */
     int32_t max_T;               /* hp.max_T = 210 */
     int32_t attention_win_size;  /* hp.attention_win_size = 3 */
     int32_t r;                   /* hp.r = 4 (SSRN upsampling = two stride-2 deconvs) */
 } dctts_hparams;
 
 /* ---- lifetime ------------------------------------------------------------------ */
-/* Replaces Graph(mode="synthesize") construction + tf.Session() (train.py:22-80, synthesize.py:26-28). */
+/* Replaces Graph(mode="synthesize") construction + tf.Session() (train.py:22-80, synthesize.py:26-28).
+ * The handle's key capacity -- the most characters (attention keys) any of its entry points takes -- is fixed here:
+ * max(192, round_up(max_N, 64)).  max_N > 512 fails with an error that names the limit. */
 int dctts_create(const dctts_hparams* hp, int device, dctts_handle* out);
 int dctts_destroy(dctts_handle h);
 const char* dctts_last_error(dctts_handle h);      /* h may be NULL: last create() error */
@@ -176,7 +178,7 @@ int dctts_train_step_ssrn(dctts_handle h, const float* mels, const float* mags, 
  * pointers, B as given to the init call.  TextEnc and the attention keys run over N rows, the other networks over T
  * frames; the L1 / binary-divergence losses average over the batch's own extent.  The guided-attention term covers the
  * window n < min(N, max_N), t < min(T, max_T) of the (max_N, max_T) weight table, divided by B min(N, max_N) min(T, max_T)
- * (train.py:91-95 pads A with -1 and cuts it to (max_N, max_T)).  N <= 192 (the attention kernels' key capacity), T is
+ * (train.py:91-95 pads A with -1 and cuts it to (max_N, max_T)).  N <= the handle's key capacity (see dctts_create), T is
  * bounded by memory only.  The activation workspace grows on demand (the device is synchronised first);
  * dctts_train_reserve pre-sizes it for steps up to (N, T) (SSRN: N is ignored).  Growth keeps the variables, gradients,
  * Adam moments and everything dctts_train_tensor reads.  At (max_N, max_T) (SSRN: the init T) the shaped steps compute
@@ -212,8 +214,10 @@ int dctts_set_tensor_path(dctts_handle h, int32_t mode);
  *   "tc_occ2" 0/1, "tc_cg2" 0/1/2, "tc_tile_pair" 0/1, "tc_mcast" 0/1, "tc_resid_tma" 0/1: tcgen05 block kernel variants
  *   "fused_ln" 0/1: graph decode, GEMM + LN in one launch;  "tc_debug" 0/1;  "decode_prof" 0/1;  "pdl" 0/1 (process-wide)
  *   "train_tc" 0..7: training GEMMs on tcgen05, bit mask 1 forward conv (+ tcgen05 attention), 2 data gradient, 4 weight gradient
- * dctts_get_option also answers "decode_available" (1 when this handle / device can run the persistent decode) and
- * "decode_max_clusters" (16-CTA clusters of the decode kernel that are co-resident on this device; 7 on a B200). */
+ * dctts_get_option also answers "decode_available" (1 when this handle / device can run the persistent decode),
+ * "key_capacity" (the most characters any entry point of this handle takes: max(192, round_up(max_N, 64)); dctts_attention,
+ * dctts_train_step_shaped and dctts_train_reserve reject a larger N) and "decode_max_clusters" (16-CTA clusters of the
+ * decode kernel that are co-resident on this device; 7 on a B200). */
 int dctts_set_option(dctts_handle h, const char* name, int32_t value);
 int dctts_get_option(dctts_handle h, const char* name, int32_t* value);
 /* Of the last dctts_text2mel_generate on the persistent decode path: frames in which a cluster had to recompute the
